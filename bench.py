@@ -365,6 +365,22 @@ def assemble_laplace3d_csr(n, kappa):
     return rowptr, cols[mask], vals[mask], ((i + j + k) & 1).astype(np.int32)
 
 
+DUMP_ENTRIES = 1 << 22  # 32 MiB of float64 over all ranks
+
+
+def dump_outputs(path, y, rank, world):
+    """Writes the chain state y after the last timed step -- what apply_richardson_dev hands back to its caller -- as
+    <path>/y.npy (float64; y_rank<r>.npy per rank for N > 1).  A state longer than its share of DUMP_ENTRIES is written as the
+    entries at a fixed sorted sample of indices (seed 0, so the same indices for the same grid), so that the dumps of two builds
+    can be compared entry for entry."""
+    os.makedirs(path, exist_ok=True)
+    v = y.cpu().numpy()
+    cap = DUMP_ENTRIES // world
+    if v.size > cap:
+        v = v[np.sort(np.random.default_rng(0).choice(v.size, cap, replace=False))]
+    np.save(os.path.join(path, "y.npy" if world == 1 else f"y_rank{rank}.npy"), v)
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -459,6 +475,8 @@ def run_b200(args):
     clk = clocks.stop() if rank == 0 else None
     value = world * args.steps * S / (ms * 1e-3)
     ms_per_sample = ms / (args.steps * S)
+    if args.dump_outputs:  # before the legs below, which advance the same chain state
+        dump_outputs(args.dump_outputs, y, rank, world)
 
     # ---- end to end through the host-pointer C-ABI call: pinned host buffers, H2D of the chain state y (b = NULL: the zero
     #      right-hand side of prior sampling is never uploaded), S samples, D2H of y, all inside the timed region ----
@@ -769,7 +787,12 @@ def main():
     ap.add_argument("--cpu-threads", type=int, default=0, help="threads of the MPIAIJ-emulation CPU baseline (0: all host cores)")
     ap.add_argument("--bytes-per-update", type=float, default=24.0, help="algorithmic bytes per DOF update of the omega = 1 colour sweep (SURVEY 8(d) K1)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the chain state after the last timed step to DIR/y.npy (a fixed sample of 2^22 entries when it is longer)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA path's outputs (--impl b200)")
     if args.levels <= 0:  # coarsen until the coarsest grid is small (SURVEY 8(d): cut at <= 33x33 + dense Cholesky; 9x9 at N = 1: the levels up to 65x65 run in one shared-memory launch)
         nx, ny = grid_of(args, max(1, args.gpus))
         args.levels = 1
