@@ -382,11 +382,22 @@ int make_csr_grid_op(pmg_ctx ctx, HostCsr &&a, int dim, const int64_t dims[3], s
 int make_csr_transfer(pmg_ctx ctx, const HostCsr &p, std::unique_ptr<Transfer> &t);
 
 // dense Cholesky sampler (chol.cu): src/pc_chols.c
+struct CholChunk { // a run of tiles [t0, t1) of one row panel (v = W b) or column panel (y = W^T v) of the packed triangle
+  int panel, t0, t1, q0, nq; // partial sums of the panel: chunks q0 .. q0 + nq - 1 of the list
+};
 struct CholSampler {
   pmg_ctx        ctx = nullptr;
   int64_t        n   = 0;
   DevBuf<double> L, LT, vcache, tmp;
   bool           use_gemv = true; // false: sequential substitution in dtrsv's order (-pc_cholsampler_b200_solve trsv)
+  // n > 4096: factor on the device, W = L^-1 kept as its lower triangle of 64 x 64 tiles (L / LT stay empty, and the
+  // one-launch V-cycle tails, which read L / LT as full matrices, are never chosen)
+  bool              packed = false;
+  int64_t           nt     = 0; // tiles per dimension
+  DevBuf<double>    tri, part;  // packed triangle; per-chunk partial sums
+  DevBuf<CholChunk> rows, cols; // work lists of the two products
+  DevBuf<unsigned>  done;       // per panel: chunks finished (the last one folds the partials and resets it)
+  double sample_bytes() const;  // compulsory bytes of one sample (two triangular products)
   int setup(pmg_ctx ctx, const HostCsr &a, const LrcData *lrc = nullptr); // lrc: factor A + B diag(S) B^T (src/pc_chols.c:119-157)
   // y = L^-T (L^-1 b + z)
   int sample(const double *b, double *y, const NoiseArgs &na);

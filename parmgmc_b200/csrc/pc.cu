@@ -747,7 +747,7 @@ static int mg_cycle_direct(pmg_pc pc, int l, const double *b, double *x, bool ze
   }
   if (!fused) {
     if (zero_guess) PMG_CUDA(cudaMemsetAsync(x, 0, (size_t)v.op->n() * sizeof(double), ctx->stream));
-    if (l == 0 && v.smp.kind == KIND_CHOL) PMG_TRY(prof_begin(pc, "L0 dense Cholesky sample", 16.0 * (double)v.smp.chol.n * (double)v.smp.chol.n, 16.0 * (double)v.smp.chol.n * (double)v.smp.chol.n));
+    if (l == 0 && v.smp.kind == KIND_CHOL) PMG_TRY(prof_begin(pc, "L0 dense Cholesky sample", v.smp.chol.sample_bytes(), v.smp.chol.sample_bytes()));
     PMG_TRY(run_level_sampler(pc, v.smp, b, x));
     if (l == 0) return prof_end(pc);
     MgLevel &c = pc->lv[l - 1];
@@ -1031,7 +1031,7 @@ static int gamgmc_setup(pmg_pc pc)
   pc->tail_top = -1;
   {
     MgLevel      &c0       = pc->lv[0];
-    if (pc->direct_cycle && L >= 3 && tail_max > 0 && c0.smp.kind == KIND_CHOL && c0.smp.its == 1 && c0.smp.chol.use_gemv && grid_tail_level_ok(c0.op)) {
+    if (pc->direct_cycle && L >= 3 && tail_max > 0 && c0.smp.kind == KIND_CHOL && c0.smp.its == 1 && c0.smp.chol.use_gemv && !c0.smp.chol.packed && grid_tail_level_ok(c0.op)) {
       int lt = 0;
       for (int l = 1; l < L - 1; ++l) {
         MgLevel &v = pc->lv[l];
@@ -1438,7 +1438,12 @@ int pmg_pc_view(pmg_pc pc, char *buf, size_t len)
     snprintf(t, sizeof t, "Number of colours: %d\n", pc->mat->op->ncolors());
     s += t;
   } else if (pc->type == "cholsampler") { // PCView_CholSampler, src/pc_chols.c:383-396
-    snprintf(t, sizeof t, "Dense Cholesky factor for sequential block of size %lld\n", (long long)pc->smp.chol.n);
+    const CholSampler &ch = pc->smp.chol;
+    snprintf(t, sizeof t, "Dense Cholesky factor for sequential block of size %lld\n", (long long)ch.n);
+    s += t;
+    if (ch.packed) snprintf(t, sizeof t, "  device factor (cuSOLVER potrf, cuBLAS trsm); samples stream the lower triangle of L^-1 in %lld tiles of 64 x 64 (%.0f bytes per sample)\n", (long long)(ch.nt * (ch.nt + 1) / 2), ch.sample_bytes());
+    else if (ch.use_gemv) snprintf(t, sizeof t, "  host factor; samples are two matrix-vector products with dense copies of L^-1\n");
+    else snprintf(t, sizeof t, "  host factor; samples are two sequential triangular solves in one CTA\n");
     s += t;
   } else {
     snprintf(t, sizeof t, "MG: type is MULTIPLICATIVE, levels=%d cycles=v\n", pc->nlevels);
@@ -1447,7 +1452,7 @@ int pmg_pc_view(pmg_pc pc, char *buf, size_t len)
       std::string d;
       pc->lv[l].op->describe(d);
       const LevelSampler &sm = pc->lv[l].smp;
-      snprintf(t, sizeof t, "  level %d: %s; sampler %s, max_it %d\n", l, d.c_str(), sm.kind == KIND_CHOL ? "cholsampler" : sm.kind == KIND_MCGIBBS ? "mcgibbs" : "sorgibbs", sm.its);
+      snprintf(t, sizeof t, "  level %d: %s; sampler %s, max_it %d\n", l, d.c_str(), sm.kind == KIND_CHOL ? (sm.chol.packed ? "cholsampler (device factor, packed L^-1)" : "cholsampler") : sm.kind == KIND_MCGIBBS ? "mcgibbs" : "sorgibbs", sm.its);
       s += t;
     }
   }

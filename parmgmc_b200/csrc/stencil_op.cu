@@ -2697,6 +2697,7 @@ bool grid_tail_smem_fits(int nlev, LevelOp *const *ops, int64_t chol_n)
 
 int grid_tail_cycle(pmg_ctx ctx, int nlev, const TailLevelSpec *lv, const CholSampler &chol, int noise_mode, uint64_t seed, const TailNoise *ns, int nns)
 {
+  if (chol.packed) PMG_FAIL(PMG_ERR_SUP, "coarse tail: the coarsest sampler keeps L^-1 packed (n = %lld), the tail reads it as a full matrix", (long long)chol.n);
   {
     bool done = false;
     PMG_TRY(grid_tail_smem_cycle(ctx, nlev, lv, chol, noise_mode, seed, ns, nns, done));
