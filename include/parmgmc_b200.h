@@ -101,7 +101,13 @@ int pmg_mat_create_csr_dist(pmg_ctx ctx, int64_t n_global, int64_t row_start, in
 /* MatCreateLRC(A, B, S, NULL): the operator A + B diag(S) B^T with B dense n x k (column-major) and S of length k, as the
  * reference's samplers receive it through MatLRCGetMats (src/mc_sor.c:565-595, src/pc_mcgibbs.c:236-244,
  * src/pc_sorgibbs.c:204-223).  A is borrowed and must outlive the result; sweeps run on A and are followed by the
- * rank-k correction y -= Bb (B^T y) of MCSORPostSOR_LRC (src/mc_sor.c:101-112). */
+ * rank-k correction y -= Bb (B^T y) of MCSORPostSOR_LRC (src/mc_sor.c:101-112).
+ * On a distributed A (this rank holds n_local < n_global rows: a slab of pmg_mat_create_laplace or pmg_mat_create_csr_dist)
+ * the call is collective and B_host holds this rank's n_local rows, column-major with leading dimension n_local (n_local = 0
+ * is allowed).  S must be bitwise identical on every rank and k the same: both are checked here, and a mismatch fails with
+ * PMG_ERR_ARG on every rank.  B^T y is folded per rank, all-gathered and summed in rank order, so every rank applies the same
+ * update and repeated runs give the same bits; the result agrees with one GPU to rounding, not bitwise.  A level that every
+ * rank holds in full never reduces across ranks.  PCWOODBURY and a cholsampler on such an operator fail with PMG_ERR_SUP. */
 int pmg_mat_create_lrc(pmg_mat A, int k, const double *B_host, const double *S_host, pmg_mat *mat);
 int pmg_mat_destroy(pmg_mat mat);
 int pmg_mat_get_size(pmg_mat mat, int64_t *n_local, int64_t *n_global, int64_t *row_start);

@@ -310,7 +310,11 @@ class Mat:
 
     @staticmethod
     def lrc(A: "Mat", B, S) -> "Mat":
-        """MatCreateLRC(A, B, S, NULL): A + B diag(S) B^T with B dense n x k (src/mc_sor.c:565-595).  A is borrowed."""
+        """MatCreateLRC(A, B, S, NULL): A + B diag(S) B^T with B dense n x k (src/mc_sor.c:565-595).  A is borrowed.
+
+        On a distributed A (a slab or row-partitioned operator) the call is collective: B holds this rank's n_local rows and
+        S must be bitwise identical on every rank (otherwise every rank raises PMGError).  B^T y is then reduced across ranks in
+        rank order, so N GPUs agree with one GPU to rounding (not bitwise); woodbury and a stand-alone cholsampler refuse it."""
         B = np.asarray(B, np.float64)
         S = np.ascontiguousarray(S, np.float64)
         if B.ndim != 2 or B.shape[0] != A.n or B.shape[1] != S.size:

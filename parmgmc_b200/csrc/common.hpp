@@ -203,26 +203,32 @@ struct SweepCoeffs {
 };
 uint64_t pmg_next_layout_version(); // process-wide counter: a new value whenever an operator is created or re-coloured
 
-// Low-rank part of an operator A + B diag(S) B^T (MATLRC) and its sweep corrections (lrc.cu).
+// Low-rank part of an operator A + B diag(S) B^T (MATLRC) and its sweep corrections (lrc.cu).  On a distributed base
+// (this rank holds n < nglobal rows) B, Bb and the vectors are this rank's rows; B^T y is folded per rank, the nranks
+// k-vectors are all-gathered and summed in rank order, so every rank applies the identical rank-k update.
 struct LevelOp;
 struct LrcData {
   pmg_ctx             ctx = nullptr;
   int64_t             n   = 0;
   int                 k   = 0, nchunks = 0;
+  bool                dist = false;                        // the base is row-distributed: B^T y and B^T C are reduced across ranks
   std::vector<double> Bh, Sh;                             // host copies (set-up)
   DevBuf<double>      B, S, sqrtS, Bb_f, Bb_b, partial, rhs; // n x k column-major; k; k; n x k (forward / backward); chunk sums; n
+  DevBuf<double>      bty_all;                            // nranks x k: slot r holds rank r's B^T y (slot 0 only on one rank)
+  DevBuf<unsigned>    ticket;                             // chunks of the current B^T y finished (the last one folds and resets it)
   bool                built       = false;
   double              omega_built = 0;
   const void         *built_for = nullptr; // base operator and its layout version the corrections were built with
   uint64_t            built_version = 0;
-  int init(pmg_ctx ctx, int64_t n, int k, const double *B_host, const double *S_host);
+  int init(pmg_ctx ctx, int64_t n, bool dist, int k, const double *B_host, const double *S_host); // collective when dist
   int build(LevelOp *base, double omega_build);                      // MCSORBuildLRCCorrection, both directions
   int prepare_rhs(const double *b, const NoiseArgs &na_eta, double *out); // out = b + B (sqrt|S| eta)
   int post(int dir, double *y);                                      // y -= Bb_dir (B^T y)
   int post_with(const double *M, double *y);                         // y -= M (B^T y), M dense n x k
   int correction_from(const std::vector<double> &C_host, DevBuf<double> &out); // out = C (S^-1 + B^T C)^-1 (src/mc_sor.c:513-535)
   int add_bsbt(const double *x, double sign, double *out);           // out += sign B (S o B^T x)
-  int bty(const double *M, const double *y);
+  int bty(const double *y);                                          // bty_all = every rank's B^T y (collective when dist)
+  int rank_update(const double *M, const double *scale, double sign, double *y); // y += sign M (sum_r bty_all[r] [o scale])
 };
 
 // An operator on one level on one device.

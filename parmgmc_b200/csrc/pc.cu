@@ -522,6 +522,7 @@ static int apply_coloring_policy(pmg_pc pc, LevelOp *op, bool is_user_mat)
 static int setup_level_sampler(pmg_ctx ctx, LevelSampler &s, LevelOp *op)
 {
   if (s.kind == KIND_CHOL) {
+    if (op->lrc_data() && op->lrc_data()->dist) PMG_FAIL(PMG_ERR_SUP, "cholsampler on a low-rank corrected operator with a row-distributed base is not supported: the exact sampler factors the whole operator on one device");
     const HostCsr *a = op->lrc_base() ? op->lrc_base()->host_csr() : op->host_csr();
     if (!a) PMG_FAIL(PMG_ERR_SUP, "cholsampler needs an assembled operator");
     return s.chol.setup(ctx, *a, op->lrc_data());
@@ -1212,6 +1213,7 @@ static int woodbury_setup(pmg_pc pc)
   pmg_ctx  ctx = pc->ctx;
   LrcData *lrc = pc->mat->op->lrc_data();
   if (!lrc || !pc->mat->base) PMG_FAIL(PMG_ERR_SUP, "PCWoodbury only supports matrices of type LRC"); // src/woodbury.c:161
+  if (lrc->dist) PMG_FAIL(PMG_ERR_SUP, "PCWoodbury on a low-rank corrected operator with a row-distributed base is not supported: its exact solver is a dense single-device solve");
   if (!pc->has("pc_woodbury_sampler") || !pc->has("pc_woodbury_solver")) PMG_FAIL(PMG_ERR_SUP, "Must provide sampler and solver"); // :149
   auto make_inner = [&](const std::string &which, pmg_pc *out) -> int {
     std::string type = pc->get("pc_woodbury_" + which, "");
